@@ -11,6 +11,7 @@ left out of the timed region.
   python bench.py --gpus N --steps K --warmup W [--model resnet50|alexnet|vgg16|googlenet|lenet] [--batch B]
                                                             (N>1: launched by torch.distributed.run, one rank per GPU)
   python bench.py --impl reference ...                      (the reference's CPU conv path + host SGD on the host cores)
+  python bench.py ... --dump-outputs DIR                    (also write what the last timed step computed, DIR/<name>.npy)
 
 Prints ONE JSON line on rank 0 (key list in DESIGN.md "Measurement").
 """
@@ -274,6 +275,8 @@ def run_ours(args):
     launches = L.b2c_launch_count() - l0
     clocks = sampler.stop() if sampler else None
     loss = t.loss()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(t, args.dump_outputs)
     # ---- end to end: every step copies the batch from pinned host memory and reads the loss back ---------------------------
     t.step(1, copy_input=True)
     barrier()
@@ -384,6 +387,25 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+DUMP_MAX_VALUES = 1 << 22     # per array: 16 MB of float32, so that a dump stays under 64 MB
+
+
+def dump_outputs(t, out_dir):
+    """What the last timed step handed back: the loss, the trainable parameters after the update and the solver's momentum
+    history (the step the update took), each flattened over the blobs in net order, as float32 .npy files.  An array larger
+    than DUMP_MAX_VALUES keeps the values at a fixed seeded sample of positions, the same for every run of the same model."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    n = t.num_params()
+    arrays = {"loss": np.array([t.loss()], np.float32),
+              "params": np.concatenate([t.get_param(i, 0) for i in range(n)]),
+              "history": np.concatenate([t.get_param(i, 2) for i in range(n)])}
+    for name, a in arrays.items():
+        if a.size > DUMP_MAX_VALUES:
+            a = a[np.sort(np.random.default_rng(1701).integers(0, a.size, DUMP_MAX_VALUES))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def time_allreduce(t, world, dev, reps=5):
     """Standalone in-place sum-allreduce of a buffer the size of the diff arena on a second communicator (nccl-tests
     convention for busbw), next to the in-step exchange that the headline already contains."""
@@ -448,7 +470,11 @@ def main():
     ap.add_argument("--lmdb", default="", help="train from this LMDB of raw uint8 Datums (tools/make_lmdb.py writes one) instead of the "
                                                "synthetic in-memory source; e2e then includes the parser threads and the database read")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the cpu_baseline leg (N = 1 only)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the loss, parameters and momentum history of the last one to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if not args.batch:
         from caffe_mpi_b200 import models
         args.batch = models.BASELINE_BATCH[args.model]

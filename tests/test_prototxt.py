@@ -1,16 +1,15 @@
 """CPU tests of the text-format prototxt reader and the Net graph builder (host/prototxt.cpp, SURVEY 8(f) rank 1).
-Part 1 uses small nets written here; part 2 reads the reference's own models/*.prototxt UNMODIFIED (skipped when the
-reference tree is not mounted, e.g. on the GPU box) and checks the derived inventories against SURVEY Appendix A and
-against caffe_mpi_b200/shapes.py, which bench.py uses where the prototxts are not available."""
+Part 1 uses small nets written here; part 2 takes the reference's own models/*.prototxt and solver.prototxt files as this
+parser read them UNMODIFIED (tests/golden/reference_models.json, written by tests/golden/make_golden.py) and checks those
+inventories against SURVEY Appendix A, against caffe_mpi_b200/shapes.py and against the nets and solvers that
+caffe_mpi_b200/models.py generates for bench.py."""
+import json
 import os
 
 import pytest
 
-from caffe_mpi_b200 import host_api as h
+from caffe_mpi_b200 import capi, host_api as h
 from caffe_mpi_b200.shapes import MODELS, EXTRA_PARAMS
-
-REF = "/root/reference"
-needs_ref = pytest.mark.skipif(not os.path.isdir(REF + "/models"), reason="reference tree not mounted")
 
 TINY = """
 name: "tiny"   # comment
@@ -93,24 +92,30 @@ def test_solver_prototxt_text():
 
 
 # ---------------------------------------------------------------------------------------- the reference's own prototxts
+def reference_models():
+    with open(os.path.join(os.path.dirname(__file__), "golden", "reference_models.json")) as f:
+        r = json.load(f)
+    assert r["conv_fields"] == [f for f, _ in capi.ConvParams._fields_]
+    return r
+
+
 REF_MODELS = [
-    # name, prototxt, kwargs, convs, fwd GF/img, learnable blobs, learnable floats   (SURVEY Appendix A)
-    ("resnet50", "models/resnet50/train_val.prototxt", {}, 53, 7.712, 161, 25557032),
-    ("alexnet", "models/bvlc_alexnet/train_val.prototxt", dict(default_size=227), 5, 1.332, 16, 60965224),
-    ("vgg16", "models/vgg16/train_val.prototxt", {}, 13, 30.693, 32, 138357544),
-    ("googlenet", "models/bvlc_googlenet/train_val.prototxt", {}, 59, 3.168, 128, 13378280),
-    ("lenet", "examples/mnist/lenet_train_test.prototxt", dict(default_channels=1, default_size=28), 2, 0.003776, 8, 431080),
+    # name, convs, fwd GF/img, learnable blobs, learnable floats   (SURVEY Appendix A)
+    ("resnet50", 53, 7.712, 161, 25557032),
+    ("alexnet", 5, 1.332, 16, 60965224),
+    ("vgg16", 13, 30.693, 32, 138357544),
+    ("googlenet", 59, 3.168, 128, 13378280),
+    ("lenet", 2, 0.003776, 8, 431080),
 ]
 
 
-@needs_ref
-@pytest.mark.parametrize("name,path,kw,nconv,gf,nblobs,nfloats", REF_MODELS, ids=[m[0] for m in REF_MODELS])
-def test_reference_prototxts_parse_unmodified(name, path, kw, nconv, gf, nblobs, nfloats):
-    n = h.Net(os.path.join(REF, path), "TRAIN", batch_override=1, **kw)
-    convs = n.conv_layers()
+@pytest.mark.parametrize("name,nconv,gf,nblobs,nfloats", REF_MODELS, ids=[m[0] for m in REF_MODELS])
+def test_reference_model_inventory(name, nconv, gf, nblobs, nfloats):
+    r = reference_models()["models"][name]
+    convs = [(nm, capi.ConvParams(*v), pd) for nm, v, pd in r["convs"]]
     assert len(convs) == nconv
-    assert sum(p.flops() for _, p, _ in convs) / 1e9 == pytest.approx(gf, rel=2e-3)
-    params = n.learnable_params()
+    assert sum(p.flops() for _, p, _ in convs) / r["batch"] / 1e9 == pytest.approx(gf, rel=2e-3)
+    params = r["params"]
     assert len(params) == nblobs and sum(c for _, c, _, _ in params) == nfloats
     assert convs[0][2] is False and all(pd for _, _, pd in convs[1:])
     if name in MODELS:     # the table bench.py uses must be exactly what the prototxt says
@@ -123,52 +128,48 @@ def test_reference_prototxts_parse_unmodified(name, path, kw, nconv, gf, nblobs,
         assert nfloats - conv_floats == EXTRA_PARAMS[name]
 
 
-@needs_ref
 def test_reference_solver_prototxts():
-    for path, policy, lr in (("models/resnet50/solver.prototxt", "poly", 0.001), ("models/bvlc_alexnet/solver.prototxt", None, None),
-                             ("models/vgg16/solver.prototxt", None, None), ("examples/mnist/lenet_solver.prototxt", "inv", 0.01)):
-        s, net = h.solver_from_prototxt(os.path.join(REF, path))
-        d = h.solver_describe(s)
-        assert net.endswith(".prototxt") and d["max_iter"] > 0
-        if policy:
-            assert d["lr_policy"] == policy and d["base_lr"] == pytest.approx(lr)
+    """The reference's solver files against the solver settings bench.py trains with (caffe_mpi_b200.models.SOLVERS)."""
+    from caffe_mpi_b200 import models
+    solvers = reference_models()["solvers"]
+    assert sorted(solvers) == ["alexnet", "lenet", "resnet50", "vgg16"]
+    for name, d in solvers.items():
+        assert d["net"].endswith(".prototxt") and d["max_iter"] > 0
+        s, net = h.solver_from_prototxt(models.SOLVERS[name], is_text=True)
+        assert h.solver_describe(s) == {k: d[k] for k in ("base_lr", "momentum", "weight_decay", "max_iter", "iter_size", "lr_policy")}
+    for name, policy, lr in (("resnet50", "poly", 0.001), ("lenet", "inv", 0.01)):
+        assert solvers[name]["lr_policy"] == policy and solvers[name]["base_lr"] == pytest.approx(lr)
 
 
 def test_generated_resnet50_has_the_reference_inventory():
-    """caffe_mpi_b200.models.resnet50_prototxt (used on the GPU box, where the reference tree is absent) against the
-    inventory of models/resnet50/train_val.prototxt: SURVEY Appendix A numbers, and layer by layer when the file is here."""
-    import os
+    """caffe_mpi_b200.models.resnet50_prototxt (what bench.py trains) against the inventory of
+    models/resnet50/train_val.prototxt: SURVEY Appendix A numbers, and layer by layer."""
     from caffe_mpi_b200 import host_api, models
     net = host_api.Net(models.resnet50_prototxt(2), "TRAIN", is_text=True)
     params = net.learnable_params()
     assert len(net.conv_layers()) == 53 and len(params) == 161
     assert sum(p[1] for p in params) == 25557032
-    ref = "/root/reference/models/resnet50/train_val.prototxt"
-    if os.path.exists(ref):
-        rnet = host_api.Net(ref, "TRAIN", batch_override=2)
-        assert net.layers() == [l for l in rnet.layers() if l[1] != "Accuracy"]
-        assert params == rnet.learnable_params()
-        a, b = net.conv_layers(), rnet.conv_layers()
-        assert [(n, bytes(p), pd) for n, p, pd in a] == [(n, bytes(p), pd) for n, p, pd in b]
+    r = reference_models()["models"]["resnet50"]
+    assert r["batch"] == 2
+    assert net.layers() == [(n, t, tuple(shp)) for n, t, shp in r["layers"] if t != "Accuracy"]
+    assert params == [tuple(p) for p in r["params"]]
+    fields = lambda p: [getattr(p, f) for f, _ in p._fields_]
+    assert [[n, fields(p), pd] for n, p, pd in net.conv_layers()] == r["convs"]
 
 
-GENERATED = [("alexnet", "models/bvlc_alexnet/train_val.prototxt", {}), ("vgg16", "models/vgg16/train_val.prototxt", {}),
-             ("googlenet", "models/bvlc_googlenet/train_val.prototxt", {}),
-             ("lenet", "examples/mnist/lenet_train_test.prototxt", dict(default_channels=1, default_size=28))]
+GENERATED = [("alexnet", {}), ("vgg16", {}), ("googlenet", {}), ("lenet", dict(default_channels=1, default_size=28))]
 
 
-@pytest.mark.parametrize("name,ref,kw", GENERATED, ids=[g[0] for g in GENERATED])
-def test_generated_prototxt_has_the_reference_inventory(name, ref, kw):
-    """caffe_mpi_b200/models.py generators (what bench.py and the GPU box use, where /root/reference does not exist) against
-    the reference's own model files: same TRAIN-phase layer list (name, type), conv shapes and learnable-parameter list."""
+@pytest.mark.parametrize("name,kw", GENERATED, ids=[g[0] for g in GENERATED])
+def test_generated_prototxt_has_the_reference_inventory(name, kw):
+    """caffe_mpi_b200/models.py generators (what bench.py trains) against the reference's own model files: same TRAIN-phase
+    layer list (name, type), conv shapes and learnable-parameter list."""
     from caffe_mpi_b200 import host_api, models
-    path = os.path.join("/root/reference", ref)
-    if not os.path.exists(path):
-        pytest.skip("reference tree not mounted")
-    r = host_api.Net(path, batch_override=8, **kw)
-    g = host_api.Net(models.PROTOTXT[name](8), is_text=True, **kw)
-    fields = lambda p: tuple(getattr(p, f) for f, _ in p._fields_)
-    assert [(n, fields(p), pd) for n, p, pd in r.conv_layers()] == [(n, fields(p), pd) for n, p, pd in g.conv_layers()]
-    assert [x[1:] for x in r.learnable_params()] == [x[1:] for x in g.learnable_params()]
-    keep = lambda net: [(n, t) for n, t, _ in net.layers() if t not in ("Accuracy", "Data", "Input")]
-    assert keep(r) == keep(g)
+    r = reference_models()["models"][name]
+    assert r["parser_defaults"] == kw
+    g = host_api.Net(models.PROTOTXT[name](r["batch"]), is_text=True, **kw)
+    fields = lambda p: [getattr(p, f) for f, _ in p._fields_]
+    assert r["convs"] == [[n, fields(p), pd] for n, p, pd in g.conv_layers()]
+    assert [x[1:] for x in r["params"]] == [list(x[1:]) for x in g.learnable_params()]
+    keep = lambda layers: [(n, t) for n, t, _ in layers if t not in ("Accuracy", "Data", "Input")]
+    assert keep(r["layers"]) == keep(g.layers())
